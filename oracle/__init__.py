@@ -20,11 +20,14 @@ Layout
 ``celerite_oracle.c`` C:     row generation, factor, solve/matmul sweeps, fused streams [A.2, A.6]
 ``dense``             numpy: dense covariance + Cholesky ground truth
 """
+import atexit
 import ctypes
 import hashlib
 import os
 import platform
+import shutil
 import subprocess
+import tempfile
 
 import numpy as np
 
@@ -52,14 +55,21 @@ def _cpu_tag():
 
 
 def build(fast=False):
-    """Compile the C oracle with gcc (per host CPU for the -march=native build)."""
+    """Compile the C oracle with gcc (per host CPU for the -march=native build) into
+    ``oracle/_build``.  In a read-only tree without a current build there, compile into a new
+    private temporary directory of this process (removed at exit), so that nothing is written
+    into the tree and no build is shared with another process or checkout."""
     name = "liboracle_fast.so" if fast else "liboracle.so"
     out = os.path.join(_HERE, "_build", _cpu_tag() if fast else "generic")
     path = os.path.join(out, name)
     src = os.path.join(_HERE, "celerite_oracle.c")
     if not os.path.exists(path) or os.path.getmtime(path) < os.path.getmtime(src):
+        if not os.access(_HERE, os.W_OK):
+            out = tempfile.mkdtemp(prefix="gadfly_b200_oracle_")
+            atexit.register(shutil.rmtree, out, True)
+            path = os.path.join(out, name)
         os.makedirs(out, exist_ok=True)
-        subprocess.check_call(["make", "-s", "-C", _HERE, f"OUT={out}", os.path.join(out, name)])
+        subprocess.check_call(["make", "-s", "-C", _HERE, f"OUT={out}", path])
     return path
 
 

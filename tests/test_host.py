@@ -311,6 +311,66 @@ def test_for_star_matches_independent_evaluation():
                 np.testing.assert_allclose(arr[sl], st[key], rtol=1e-12, err_msg=f"batched {name} {key}")
 
 
+def test_bench_dump_output_sample_dtype_and_size(tmp_path):
+    """bench.py --dump-outputs: an array longer than DUMP_ELEMS is stored as the same seeded sample of
+    its elements whatever its type (numpy / torch) and shape, every array in float64, and the twelve
+    arrays the bench writes stay under 64 MB."""
+    import torch
+    import bench
+    big = np.arange(3 * bench.DUMP_ELEMS, dtype=np.float64) * 0.5
+    bench.dump_output(str(tmp_path / "a"), "x", big)
+    bench.dump_output(str(tmp_path / "b"), "x", torch.as_tensor(big).reshape(3, -1))
+    a, b = np.load(tmp_path / "a" / "x.npy"), np.load(tmp_path / "b" / "x.npy")
+    assert a.dtype == np.float64 and a.shape == (bench.DUMP_ELEMS,)
+    np.testing.assert_array_equal(a, b)
+    assert np.all(np.diff(a) > 0) and np.all(np.isin(a, big))        # distinct input elements, in order
+    assert 12 * os.path.getsize(tmp_path / "a" / "x.npy") < 64 << 20
+    bench.dump_output(str(tmp_path / "a"), "status", torch.tensor([0, 2, -1], dtype=torch.int32))
+    s = np.load(tmp_path / "a" / "status.npy")
+    assert s.dtype == np.float64 and s.tolist() == [0.0, 2.0, -1.0]
+
+
+def test_bench_rejects_bad_arguments(monkeypatch):
+    import bench
+    for argv in (["--steps", "0"], ["--impl", "reference", "--dump-outputs", "d"]):
+        monkeypatch.setattr(sys, "argv", ["bench.py"] + argv)
+        with pytest.raises(SystemExit):
+            bench.parse()
+    monkeypatch.setattr(sys, "argv", ["bench.py", "--steps", "5", "--dump-outputs", "d"])
+    a = bench.parse()
+    assert a.steps == 5 and a.dump_outputs == "d"
+
+
+def test_oracle_build_in_read_only_tree_is_private(tmp_path, monkeypatch):
+    """Without a current build in oracle/_build and without write access to oracle/, the oracle is
+    compiled into a new private temporary directory per call: nothing goes into the tree, and no
+    build is shared with another process or checkout."""
+    import shutil
+    import oracle
+    tree = tmp_path / "oracle"
+    tree.mkdir()
+    for f in ("Makefile", "celerite_oracle.c"):
+        shutil.copy(os.path.join(ROOT, "oracle", f), tree / f)
+    monkeypatch.setattr(oracle, "_HERE", str(tree))
+    tree.chmod(0o555)
+    if os.getuid() == 0:                        # permission bits do not bind root
+        monkeypatch.setattr(oracle.os, "access", lambda path, mode: False)
+    paths = []
+    try:
+        paths = [oracle.build(fast=False), oracle.build(fast=False)]
+        assert paths[0] != paths[1]
+        for p in paths:
+            d = os.path.dirname(p)
+            assert not p.startswith(str(tree)) and os.stat(d).st_mode & 0o077 == 0
+            assert os.stat(d).st_uid == os.getuid()
+            ctypes.CDLL(p).orc_max_threads()
+        assert sorted(os.listdir(tree)) == ["Makefile", "celerite_oracle.c"]
+    finally:
+        tree.chmod(0o755)
+        for p in paths:
+            shutil.rmtree(os.path.dirname(p), ignore_errors=True)
+
+
 def test_bin_ranges_match_host_binning():
     """The index ranges handed to the device binning kernel are scipy.stats.binned_statistic's bins
     (what ``bin_power_spectrum`` uses on the host): every point in exactly one bin, the last edge
