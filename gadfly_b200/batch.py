@@ -136,7 +136,12 @@ def sample(kernels, t, diag=None, lengths=None, normals=None, seed=0, seq0=0, so
     """One GP draw per unit: ``x = L (sqrt(d) o n)``.  ``normals=None`` draws n on the device
     from Philox4x32-10 keyed by ``seed`` and the global unit index ``seq0 + b``
     (reproducible on the host with :mod:`gadfly_b200.philox`).  ``subtract_mean`` applies the
-    reference's per-draw mean subtraction (gadfly/gp.py:392)."""
+    reference's mean subtraction (gadfly/gp.py:392): over the draw's samples for one draw, over the
+    realisations at each time stamp for ``size`` of them.  It needs the draws on the host, so it
+    cannot be combined with ``FLAG_ASYNC`` (the buffer is written after this returns)."""
+    from .solver import FLAG_ASYNC
+    if subtract_mean and (flags & FLAG_ASYNC):
+        raise ValueError("subtract_mean needs the draws: pass subtract_mean=False with FLAG_ASYNC")
     kb = _as_batch(kernels)
     geom = _geometry(kb, t, lengths)
     solver = solver or default_solver()
@@ -151,9 +156,10 @@ def sample(kernels, t, diag=None, lengths=None, normals=None, seed=0, seq0=0, so
             return x, status
         rows = [x[k * geom.n_off[b]:k * geom.n_off[b + 1]].reshape(k, -1) for b in range(kb.B)]
         if subtract_mean:
+            # celerite2's sample(size=k) returns [k, N]; the reference subtracts result.mean(axis=0)
             for r in rows:
                 if r.size:
-                    r -= r.mean(axis=1, keepdims=True)
+                    r -= r.mean(axis=0, keepdims=True)
         return (np.stack(rows) if lengths is None else rows), status
     x, logdet, status = solver.sample(kb, geom, t, diag, normals, seed=seed, seq0=seq0, out=out,
                                       flags=flags)

@@ -122,6 +122,7 @@ struct gf_context {
     int sm_count = 0;
     double fp64_flops = 0.0;
     int64_t launches = 0;
+    int scan_path = GF_PATH_NONE;        // kernel of the most recent scan launch (gf_last_scan_path)
     bool timed = false;
     std::string err;
     gf::FftPlan *fft = nullptr;
@@ -481,22 +482,27 @@ int run_scan(gf_handle h, int mode, int64_t B, const int64_t *n_off, const int64
             GF_CUDA(h, reserve(h, S_WIDE, gf::scan_wide_state_bytes(grid), &state));
             GF_CUDA(h, gf::launch_scan_wide(mode, A, grid, (double *)state, h->stream));
             h->launches += 1;
+            h->scan_path = GF_PATH_WIDE;
         } else if ((flags & GF_FLAG_BLOCKED) && !ref && gf::scan_blk_supports(mode, g.jmax)) {
             GF_CUDA(h, gf::launch_scan_blk(mode, A, h->sm_count, h->stream));
             h->launches += 1;
+            h->scan_path = GF_PATH_BLOCKED;
         } else if (ref) {
             int grid = (int)std::min<int64_t>(B, (int64_t)h->sm_count);
             GF_CUDA(h, gf::launch_scan_ref(mode, A, grid, h->stream));
             h->launches += 1;
+            h->scan_path = GF_PATH_REF;
         } else if (!(flags & GF_FLAG_WIDE_KERNEL) && gf::scan_small_supports(mode, g.jmax)) {
             // every sequence of the batch is narrow (J <= 32): one warp per sequence
             int n = 0;
             GF_CUDA(h, gf::launch_scan_small(mode, A, g.jmax, h->sm_count, h->stream, &n));
             h->launches += n;
+            h->scan_path = GF_PATH_SMALL;
         } else {
             int n = 0;
             GF_CUDA(h, gf::launch_scan_fast(mode, A, g.jmax, h->sm_count, h->stream, &n));
             h->launches += n;
+            h->scan_path = GF_PATH_FAST;
         }
     }
 
@@ -640,6 +646,8 @@ int gf_device_info(gf_handle h, int *sm_count, double *fp64_flops, int measure)
 }
 
 int64_t gf_launch_count(gf_handle h) { return h ? h->launches : 0; }
+
+int gf_last_scan_path(gf_handle h) { return h ? h->scan_path : GF_E_ARG; }
 
 float gf_last_kernel_ms(gf_handle h)
 {

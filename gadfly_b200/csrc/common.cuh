@@ -104,10 +104,13 @@ __device__ __forceinline__ void sincos_cw(double x, double *sn, double *cs)
 }
 
 // log-determinant accumulation without a log per step: a positive normal pivot is split into its
-// mantissa in [1, 2) (multiplied into `prod`, at most 2^8 between flushes) and its binary exponent
-// (summed as an integer), so that no product of pivots can overflow or underflow whatever the
-// flux scale; sum log d = sum log(prod) + ln 2 * esum.  (Subnormal pivots keep their value: their
-// exponent field is 0 and they are multiplied in unscaled.)
+// mantissa in [1, 2) (multiplied into `prod`) and its binary exponent (summed as an integer), so
+// that the product cannot overflow or underflow whatever the flux scale; sum log d = sum log(prod)
+// + ln 2 * esum.  The callers flush `prod` into a log and the int `esum` into a long long every
+// 8 (scan_small) or 32 (scan_blk) pivots: a sequence's exponent sum can pass 2^31.  scan_fast
+// splits its pivots the same way but adds ln 2 * exponent to its log sum directly (no counter in
+// its register-bound chain); scan_ref and scan_wide take one log per pivot.  (Subnormal pivots
+// keep their value here: their exponent field is 0 and they are multiplied in unscaled.)
 __device__ __forceinline__ void logdet_push(double d, double &prod, int &esum)
 {
     const int hi = __double2hiint(d);

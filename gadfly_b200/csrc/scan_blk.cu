@@ -237,7 +237,8 @@ __device__ __forceinline__ void blk_chain_loop(FastSmem &sm, BlkSmem &ex, const 
     bar_arrive(BAR_S2, BLK_THREADS);                  // "the update before block 0": nothing
     double rdp[KB] = {0.0, 0.0, 0.0, 0.0};            // 1 / d of the previous block
     double logsum = 0.0, prod = 1.0, quad = 0.0;
-    int esum = 0;
+    int esum32 = 0;                                   // pivot exponents since the last flush of prod
+    long long esum = 0;                               // (N |exponent| passes 2^31 at large flux scales)
     int32_t fail = 0;
     bool dead = false;
 #ifdef GF_BLK_TIMING
@@ -457,11 +458,11 @@ __device__ __forceinline__ void blk_chain_loop(FastSmem &sm, BlkSmem &ex, const 
 #pragma unroll
             for (int i = 0; i < KB; ++i)
                 if (i < good) {
-                    logdet_push(dd[i], prod, esum);
+                    logdet_push(dd[i], prod, esum32);
                     if (MODE == MODE_LOGLIKE) quad = fma(zz[i] * zz[i], rd[i], quad);
                     else A.out_x[n0g + n0 + i] = xx[i];
                 }
-            if ((n1 & 31) < KB || !more) { logsum += log(prod); prod = 1.0; }
+            if ((n1 & 31) < KB || !more) { logsum += log(prod); prod = 1.0; esum += esum32; esum32 = 0; }
             if (bad >= 0) sm.stop = n0 + bad;         // the producer keeps only the hand-shake going
         }
         if (bad >= 0) { fail = n0 + bad + 1; dead = true; }
@@ -507,7 +508,7 @@ __device__ __forceinline__ void blk_chain_loop(FastSmem &sm, BlkSmem &ex, const 
     }
     if (ht == 0) {
         if (prod != 1.0) logsum += log(prod);
-        A.logdet[b] = logdet_total(logsum, 1.0, esum);
+        A.logdet[b] = logdet_total(logsum, 1.0, esum + esum32);
         if (MODE == MODE_LOGLIKE && A.quad) A.quad[b] = quad;
         A.status[b] = fail;
     }

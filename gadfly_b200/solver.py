@@ -36,6 +36,11 @@ FLAG_SHARED_Y = 4
 FLAG_WIDE_KERNEL = 8
 FLAG_BLOCKED = 16
 
+# scan kernel that served a call (gf_last_scan_path; include/gadfly_b200.h GF_PATH_*)
+PATH_NONE, PATH_FAST, PATH_SMALL, PATH_REF, PATH_WIDE, PATH_BLOCKED = -1, 0, 1, 2, 3, 4
+PATH_NAMES = {PATH_NONE: "none", PATH_FAST: "scan_fast", PATH_SMALL: "scan_small", PATH_REF: "scan_ref",
+              PATH_WIDE: "scan_wide", PATH_BLOCKED: "scan_blk"}
+
 _HERE = os.path.dirname(os.path.abspath(__file__))
 _LIBNAME = "libgadfly_b200.so"
 
@@ -77,6 +82,7 @@ _SIGNATURES = {
                                       ctypes.POINTER(ctypes.c_double), ctypes.c_int]),
     "gf_launch_count": (ctypes.c_int64, [ctypes.c_void_p]),
     "gf_last_kernel_ms": (ctypes.c_float, [ctypes.c_void_p]),
+    "gf_last_scan_path": (ctypes.c_int, [ctypes.c_void_p]),
     "gf_loglike_batched": (ctypes.c_int, [
         ctypes.c_void_p, ctypes.c_int64, _i64p, _i64p, _i64p, _f64p, ctypes.c_int64, _f64p, _f64p,
         _f64p, _f64p, _f64p, _f64p, _i32p, ctypes.c_uint32]),
@@ -378,6 +384,12 @@ class Solver:
     @property
     def last_kernel_ms(self):
         return float(self._lib.gf_last_kernel_ms(self._h))
+
+    def last_scan_path(self):
+        """Name of the scan kernel that served the most recent scan launch on this handle
+        (``"scan_fast"``, ``"scan_small"``, ``"scan_ref"``, ``"scan_wide"``, ``"scan_blk"``), or
+        ``"none"`` before the first one."""
+        return PATH_NAMES[int(self._lib.gf_last_scan_path(self._h))]
 
     def device_info(self, measure=False):
         sm = ctypes.c_int()

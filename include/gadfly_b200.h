@@ -112,6 +112,18 @@ int64_t gf_launch_count(gf_handle h);
 /* device time [ms] of the most recent scan / psd kernel launch, from CUDA events recorded
  * on the handle's stream around the launch (valid after the call returned / synchronised) */
 float gf_last_kernel_ms(gf_handle h);
+/* which scan kernel served the most recent scan launch of the handle (gf_loglike_batched,
+ * gf_sample_batched, gf_factor_batched and the factor scan of gf_*_multi): one of GF_PATH_*,
+ * GF_PATH_NONE before the first scan launch (a call with B = 0 launches nothing) */
+enum {
+    GF_PATH_NONE = -1,
+    GF_PATH_FAST = 0,      /* csrc/scan_fast.cu: register-resident state, J <= GF_MAX_J */
+    GF_PATH_SMALL = 1,     /* csrc/scan_small.cu: one warp per sequence, every J <= 32 */
+    GF_PATH_REF = 2,       /* csrc/scan_ref.cu: GF_FLAG_REFERENCE_ORDER */
+    GF_PATH_WIDE = 3,      /* csrc/scan_wide.cu: some J > GF_MAX_J */
+    GF_PATH_BLOCKED = 4    /* csrc/scan_blk.cu: GF_FLAG_BLOCKED */
+};
+int gf_last_scan_path(gf_handle h);
 
 /* ---- K1: fused factor + forward solve -> log-likelihood pieces ---------------------
  * Replaces, per sequence: celerite2 GaussianProcess.compute (driver.factor; reference

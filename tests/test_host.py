@@ -198,6 +198,14 @@ def test_gp_usage_before_compute_raises(solar_kernel):
         gp.compute(np.zeros((2, 2)))
 
 
+def test_sample_mean_subtraction_refuses_async(solar_kernel):
+    """batch.sample subtracts the mean on the host: with FLAG_ASYNC the draws are not there yet."""
+    t = np.arange(16) * 6e-5
+    for size in (None, 3):
+        with pytest.raises(ValueError, match="FLAG_ASYNC"):
+            batch.sample([solar_kernel], t, size=size, flags=solver.FLAG_ASYNC)
+
+
 def test_power_spectrum_fft_normalisation():
     rng = np.random.default_rng(0)
     t = np.arange(4096) / 1440.0                # 1-min cadence in days
