@@ -2,7 +2,8 @@
 //
 // Everything here is host-side plumbing: pointer classification and staging, batch
 // descriptors, the heaviest-first work order, launch bookkeeping.  The arithmetic is in
-// scan_fast.cu / scan_ref.cu (O(N J^2) scans), sweep.cu (O(N J) sweeps) and psd.cu.
+// scan_fast.cu / scan_small.cu / scan_blk.cu / scan_ref.cu (O(N J^2) scans), sweep.cu (O(N J)
+// sweeps) and psd.cu.
 #include "../../include/gadfly_b200.h"
 #include "common.cuh"
 
@@ -17,14 +18,12 @@
 #include <vector>
 
 namespace gf {
-cudaError_t launch_scan_ref(int mode, const ScanArgs &args, int grid, cudaStream_t stream);
+size_t scan_ref_scratch_bytes(int jmax, int grid);
+cudaError_t launch_scan_ref(int mode, const ScanArgs &args, int jmax, int grid, double *scratch,
+                            cudaStream_t stream);
 cudaError_t launch_scan_fast(int mode, const ScanArgs &args, int jmax, int sm_count,
                              cudaStream_t stream, int *launches);
-bool scan_fast_supports(int mode, int jmax);
 bool scan_small_supports(int mode, int jmax);
-bool scan_wide_supports(int jmax);
-size_t scan_wide_state_bytes(int grid);
-cudaError_t launch_scan_wide(int mode, const ScanArgs &args, int grid, double *state, cudaStream_t stream);
 cudaError_t launch_scan_small(int mode, const ScanArgs &args, int jmax, int sm_count,
                               cudaStream_t stream, int *launches);
 cudaError_t launch_sweep(int op, int64_t B, const int64_t *n_off, const int64_t *t_off,
@@ -474,24 +473,20 @@ int run_scan(gf_handle h, int mode, int64_t B, const int64_t *n_off, const int64
     GF_CUDA(h, begin_kernel(h));
     {
         Timer timer(h);
-        const bool ref = (flags & GF_FLAG_REFERENCE_ORDER) || !gf::scan_fast_supports(mode, g.jmax);
-        if (g.jmax > GF_MAX_J) {
-            // wider than the register-resident kernels take: state in L2-resident global scratch
+        if ((flags & GF_FLAG_REFERENCE_ORDER) || g.jmax > GF_MAX_J) {
+            // reference order; a state wider than the register-resident kernels take (J > 176) lives
+            // in L2-resident global scratch whatever the flags
             const int grid = (int)std::min<int64_t>(B, (int64_t)h->sm_count);
+            const size_t bytes = gf::scan_ref_scratch_bytes(g.jmax, grid);
             void *state = nullptr;
-            GF_CUDA(h, reserve(h, S_WIDE, gf::scan_wide_state_bytes(grid), &state));
-            GF_CUDA(h, gf::launch_scan_wide(mode, A, grid, (double *)state, h->stream));
+            if (bytes) GF_CUDA(h, reserve(h, S_WIDE, bytes, &state));
+            GF_CUDA(h, gf::launch_scan_ref(mode, A, g.jmax, grid, (double *)state, h->stream));
             h->launches += 1;
-            h->scan_path = GF_PATH_WIDE;
-        } else if ((flags & GF_FLAG_BLOCKED) && !ref && gf::scan_blk_supports(mode, g.jmax)) {
+            h->scan_path = bytes ? GF_PATH_WIDE : GF_PATH_REF;
+        } else if ((flags & GF_FLAG_BLOCKED) && gf::scan_blk_supports(mode, g.jmax)) {
             GF_CUDA(h, gf::launch_scan_blk(mode, A, h->sm_count, h->stream));
             h->launches += 1;
             h->scan_path = GF_PATH_BLOCKED;
-        } else if (ref) {
-            int grid = (int)std::min<int64_t>(B, (int64_t)h->sm_count);
-            GF_CUDA(h, gf::launch_scan_ref(mode, A, grid, h->stream));
-            h->launches += 1;
-            h->scan_path = GF_PATH_REF;
         } else if (!(flags & GF_FLAG_WIDE_KERNEL) && gf::scan_small_supports(mode, g.jmax)) {
             // every sequence of the batch is narrow (J <= 32): one warp per sequence
             int n = 0;

@@ -109,7 +109,7 @@ __device__ __forceinline__ void sincos_cw(double x, double *sn, double *cs)
 // + ln 2 * esum.  The callers flush `prod` into a log and the int `esum` into a long long every
 // 8 (scan_small) or 32 (scan_blk) pivots: a sequence's exponent sum can pass 2^31.  scan_fast
 // splits its pivots the same way but adds ln 2 * exponent to its log sum directly (no counter in
-// its register-bound chain); scan_ref and scan_wide take one log per pivot.  (Subnormal pivots
+// its register-bound chain); scan_ref.cu takes one log per pivot.  (Subnormal pivots
 // keep their value here: their exponent field is 0 and they are multiplied in unscaled.)
 __device__ __forceinline__ void logdet_push(double d, double &prod, int &esum)
 {

@@ -1221,12 +1221,6 @@ cudaError_t launch_mode(const ScanArgs &args, int grid, cudaStream_t stream)
 }  // namespace
 
 #ifndef GF_SCAN_FAST_AS_HEADER   // scan_blk.cu includes this file for the producer warp and the tile map
-bool scan_fast_supports(int mode, int jmax)
-{
-    (void)mode;
-    return jmax <= JP_MAX;
-}
-
 cudaError_t launch_scan_fast(int mode, const ScanArgs &args, int jmax, int sm_count,
                              cudaStream_t stream, int *launches)
 {

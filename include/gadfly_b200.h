@@ -119,8 +119,8 @@ enum {
     GF_PATH_NONE = -1,
     GF_PATH_FAST = 0,      /* csrc/scan_fast.cu: register-resident state, J <= GF_MAX_J */
     GF_PATH_SMALL = 1,     /* csrc/scan_small.cu: one warp per sequence, every J <= 32 */
-    GF_PATH_REF = 2,       /* csrc/scan_ref.cu: GF_FLAG_REFERENCE_ORDER */
-    GF_PATH_WIDE = 3,      /* csrc/scan_wide.cu: some J > GF_MAX_J */
+    GF_PATH_REF = 2,       /* csrc/scan_ref.cu, state in registers: GF_FLAG_REFERENCE_ORDER */
+    GF_PATH_WIDE = 3,      /* csrc/scan_ref.cu, state in L2-resident scratch: some J > GF_MAX_J */
     GF_PATH_BLOCKED = 4    /* csrc/scan_blk.cu: GF_FLAG_BLOCKED */
 };
 int gf_last_scan_path(gf_handle h);

@@ -1,6 +1,6 @@
-"""Conformance of every scan kernel (csrc/scan_fast.cu, scan_small.cu, scan_ref.cu, scan_wide.cu,
-scan_blk.cu) to relations that hold EXACTLY, independent of any reference implementation, plus the
-dispatch and length edges against the oracle.
+"""Conformance of every scan path (csrc/scan_fast.cu, scan_small.cu, scan_blk.cu, and scan_ref.cu with
+its register store "scan_ref" and its L2 store "scan_wide") to relations that hold EXACTLY, independent
+of any reference implementation, plus the dispatch and length edges against the oracle.
 
 * Amplitude: a', b', ddiag and diag times s = 2^e, y times 2^(e/2).  Every product and sum of the
   recurrence scales by a power of two, so IEEE rounding commutes with it: quad and the samples are
@@ -15,6 +15,7 @@ dispatch and length edges against the oracle.
 * Batch placement: the scans are persistent (CTAs / warps claim sequences from a queue and reuse
   shared memory, ring phases and flags between sequences); a sequence's result must not depend on
   which sequences ran before it on the same CTA.
+* State stores: scan_ref.cu's two stores give a J <= 176 sequence the same bits.
 
 Every case asserts which kernel served it (``Solver.last_scan_path``): a path added to ``PATHS`` is
 covered by every parametrised case below."""
@@ -651,3 +652,37 @@ def test_sample_size_k_matches_oracle(solver, kern, path):
         scale = np.max(np.abs(ogp.dot_tril(n)))
         assert np.max(np.abs(rows[b] - ref)) <= RTOL * scale, b
         np.testing.assert_allclose(rows[b].mean(axis=0), 0.0, atol=1e-12 * scale)
+
+
+# ---- h. the two state stores of the reference-order kernel ---------------------------------------
+@pytest.mark.parametrize("mode", ["loglike", "sample", "philox", "factor"])
+@pytest.mark.parametrize("J", [100, 172])
+def test_reference_order_state_stores_agree(solver, kern, J, mode):
+    """scan_ref_kernel keeps the J x J state in registers ("scan_ref") or, in a batch with a kernel
+    wider than 176, in L2-resident scratch ("scan_wide").  Both stores run the same per-tile
+    expressions and folds in the same order, so a J <= 176 sequence run alone under
+    FLAG_REFERENCE_ORDER and beside a J = 300 kernel gives the same bits.  ("philox": sampling with
+    the normals drawn in the kernel; the sequence is index 0 of both batches.)"""
+    N, n2 = 3000, 64
+    k, wide = kern(J), kern(300)
+    t = _gappy(N, 23)
+    dg = 1e-3 * _k0(k) * (1.0 + np.random.default_rng(24).uniform(0.0, 2.0, N))
+    dg2 = np.full(n2, 1e-3 * _k0(wide))
+    v = np.random.default_rng(25).standard_normal(N + n2)
+    scan_mode = "sample" if mode == "philox" else mode
+    data = {"loglike": np.concatenate([v[:N] * np.sqrt(_k0(k)), v[N:] * np.sqrt(_k0(wide))]),
+            "sample": v, "philox": None, "factor": None}[mode]
+    alone = _run(solver, "scan_ref", scan_mode, KernelBatch([k]), Geometry.shared_t(1, N), t,
+                 None if data is None else data[:N], dg)
+    kb, geom = KernelBatch([k, wide]), Geometry.ragged([N, n2])
+    both = _run(solver, "scan_wide", scan_mode, kb, geom, np.concatenate([t, _gappy(n2, 26)]), data,
+                np.concatenate([dg, dg2]))
+    assert alone["status"][0] == 0 and both["status"].tolist() == [0, 0]
+    assert both["logdet"][0] == alone["logdet"][0]
+    if mode == "loglike":
+        assert both["quad"][0] == alone["quad"][0]
+    elif scan_mode == "sample":
+        np.testing.assert_array_equal(both["x"][:N], alone["x"])
+    else:
+        np.testing.assert_array_equal(both["d"][:N], alone["d"])
+        np.testing.assert_array_equal(both["W"][:N * J], alone["W"])
