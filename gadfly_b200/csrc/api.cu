@@ -1,13 +1,15 @@
 // C ABI of the gadfly_b200 CUDA library (see include/gadfly_b200.h for the contract).
 //
 // Everything here is host-side plumbing: pointer classification and staging, batch
-// descriptors, the heaviest-first work order, launch bookkeeping.  The arithmetic is in
+// descriptors, the heaviest-first work order, launch bookkeeping.  Every entry point does its
+// staging, launches and copies back through one `Call`.  The arithmetic is in
 // scan_fast.cu / scan_small.cu / scan_blk.cu / scan_ref.cu (O(N J^2) scans), sweep.cu (O(N J)
 // sweeps) and psd.cu.
 #include "../../include/gadfly_b200.h"
 #include "common.cuh"
 
 #include <algorithm>
+#include <cassert>
 #include <cmath>
 #include <cstdio>
 #include <cstring>
@@ -116,7 +118,7 @@ struct gf_context {
     cudaEvent_t ev_in = nullptr, ev_k = nullptr, ev_ext = nullptr;
     bool in_dirty = false;
     uint64_t stamp = 0;
-    std::vector<Buf *> touched;          // staging buffers the kernel of the current call uses
+    std::vector<Buf *> touched;          // staging buffers the kernels of the current call use
     cudaEvent_t ev0 = nullptr, ev1 = nullptr;
     int sm_count = 0;
     double fp64_flops = 0.0;
@@ -147,8 +149,6 @@ namespace {
 struct Guard {
     int prev = -1;
     explicit Guard(int dev) { cudaGetDevice(&prev); if (prev != dev) cudaSetDevice(dev); }
-    // entry points that stage buffers: also drop what a failed earlier call may have left behind
-    explicit Guard(gf_handle h) : Guard(h->device) { h->touched.clear(); }
     ~Guard() { if (prev >= 0) cudaSetDevice(prev); }
 };
 
@@ -277,27 +277,25 @@ cudaError_t stage_in(gf_handle h, int slot, const T *src, size_t count, const T 
 }
 
 // Output that may live on the host: device pointer now, copy back later.
-template <typename T>
 struct Out {
-    T *user = nullptr;
-    T *dev = nullptr;
-    size_t count = 0;
+    void *user = nullptr;
+    void *dev = nullptr;
+    size_t bytes = 0;
     bool host = false;
     bool pageable = false;
     Buf *buf = nullptr;
 };
 
-template <typename T>
-cudaError_t stage_out(gf_handle h, int slot, T *dst, size_t count, Out<T> *o)
+cudaError_t stage_out(gf_handle h, int slot, void *dst, size_t bytes, Out *o)
 {
-    o->user = dst; o->count = count; o->host = false; o->pageable = false; o->dev = dst; o->buf = nullptr;
-    if (!dst || count == 0) return cudaSuccess;
+    *o = Out{dst, dst, bytes};
+    if (!dst || bytes == 0) return cudaSuccess;
     const int kind = pointer_kind(dst);
     if (kind == P_DEVICE) return cudaSuccess;
     o->pageable = kind == P_PAGEABLE;
-    cudaError_t e = acquire(h, slot, count * sizeof(T), h->stream, &o->buf);
+    cudaError_t e = acquire(h, slot, bytes, h->stream, &o->buf);
     if (e != cudaSuccess) return e;
-    o->dev = (T *)o->buf->p;
+    o->dev = o->buf->p;
     o->host = true;
     return cudaSuccess;
 }
@@ -312,8 +310,9 @@ cudaError_t begin_kernel(gf_handle h)
     return cudaStreamWaitEvent(h->stream, h->ev_in, 0);
 }
 
-// The kernel(s) of this call are launched: stamp the staging buffers they use, and let the
-// copy-out stream wait for them.
+// The kernel(s) of this call are launched: stamp the staging buffers the call has used so far, and
+// let the copy-out stream wait for them.  The list is kept, so that a later kernel phase of the same
+// call stamps again what it shares with an earlier one.
 cudaError_t end_kernel(gf_handle h)
 {
     cudaError_t e = cudaEventRecord(h->ev_k, h->stream);
@@ -325,15 +324,13 @@ cudaError_t end_kernel(gf_handle h)
         b->pending = true;
         b->stamp = h->stamp;
     }
-    h->touched.clear();
     return cudaStreamWaitEvent(h->s_out, h->ev_k, 0);
 }
 
-template <typename T>
-cudaError_t finish_out(gf_handle h, const Out<T> &o)
+cudaError_t finish_out(gf_handle h, const Out &o)
 {
-    if (!o.host || !o.user || o.count == 0) return cudaSuccess;
-    const size_t bytes = o.count * sizeof(T);
+    if (!o.host || !o.user || o.bytes == 0) return cudaSuccess;
+    const size_t bytes = o.bytes;
     void *dst = o.user;
     size_t ring_end = 0;
     char *pinned = (o.pageable && bytes <= BOUNCE_MAX) ? bounce_alloc(h, bytes, &ring_end) : nullptr;
@@ -358,6 +355,129 @@ cudaError_t finish_call(gf_handle h, uint32_t flags)
     e = cudaStreamSynchronize(h->s_out);
     if (e == cudaSuccess) flush_deferred(h, h->out_seq);
     return e;
+}
+
+// One entry point's work on the handle, in the order its steps are called: inputs, outputs and
+// scratch staged in their slots (the order of the in() calls is the order of the H2D copies), one or
+// more kernel phases, then finish(): the copies back in the order the outputs were registered, and
+// the wait for them unless GF_FLAG_ASYNC.  The first CUDA error is kept; every later step does
+// nothing, and finish() reports it.
+//
+// Staged outputs are not put on `touched`: finish() stamps each of them with its copy back, which the
+// copy-out stream issues after the call's kernels.  Inputs and scratch are stamped at the end of every
+// kernel phase.
+class Call {
+public:
+    gf_handle const h;
+
+    Call(gf_handle h_, uint32_t flags) : h(h_), flags_(flags), guard_(h_->device)
+    {
+        h->touched.clear();   // the buffers of earlier calls (stamped, unless such a call failed)
+    }
+
+    bool ok() const { return err_ == cudaSuccess; }
+    void check(cudaError_t e, const char *what)
+    {
+        if (ok() && e != cudaSuccess) { err_ = e; what_ = what; }
+    }
+
+    // device pointer of an input (nullptr once the call has failed)
+    template <typename T>
+    const T *in(int slot, const T *src, size_t count)
+    {
+        const T *dev = nullptr;
+        if (ok()) check(stage_in(h, slot, src, count, &dev), "stage_in");
+        return ok() ? dev : nullptr;
+    }
+
+    // device pointer the kernel writes an output to; a host output is copied back by finish()
+    template <typename T>
+    T *out(int slot, T *dst, size_t count)
+    {
+        if (!ok()) return nullptr;
+        Out o;
+        check(stage_out(h, slot, dst, count * sizeof(T), &o), "stage_out");
+        if (!ok()) return nullptr;
+        if (o.host) {
+            assert(n_outs_ < MAX_OUTS);
+            outs_[n_outs_++] = o;
+        }
+        return (T *)o.dev;
+    }
+
+    // device scratch of the kernels (nullptr once the call has failed)
+    void *scratch(int slot, size_t bytes)
+    {
+        void *p = nullptr;
+        if (ok()) check(reserve(h, slot, bytes, &p), "reserve");
+        return ok() ? p : nullptr;
+    }
+
+    // One kernel phase: `launch` issues the kernels on the compute stream once every input staged so
+    // far has arrived (its errors go to check(), through GF_STEP) and returns how many it launched.
+    template <typename F>
+    void kernels(bool timed, F launch)
+    {
+        if (!ok()) return;
+        check(begin_kernel(h), "begin_kernel");
+        if (!ok()) return;
+        if (timed) cudaEventRecord(h->ev0, h->stream);
+        const int64_t launches = launch();
+        if (timed) { cudaEventRecord(h->ev1, h->stream); h->timed = true; }
+        if (!ok()) return;
+        h->launches += launches;
+        check(end_kernel(h), "end_kernel");
+    }
+
+    int finish()
+    {
+        for (int i = 0; i < n_outs_ && ok(); ++i) check(finish_out(h, outs_[i]), "finish_out");
+        if (ok()) check(finish_call(h, flags_), "finish_call");
+        return ok() ? GF_OK : fail(h, (int)err_, what_);
+    }
+
+private:
+    static constexpr int MAX_OUTS = 5;
+    uint32_t flags_;
+    Guard guard_;
+    cudaError_t err_ = cudaSuccess;
+    const char *what_ = nullptr;
+    Out outs_[MAX_OUTS];
+    int n_outs_ = 0;
+};
+
+// a CUDA call an entry point makes itself: skipped once the call has failed, its error kept by the call
+#define GF_STEP(c, expr) do { if ((c).ok()) (c).check((expr), #expr); } while (0)
+
+// max over b of w_off[b] + N_b J_b: the length of a W laid out by w_off
+int64_t w_extent(int64_t B, const int64_t *n_off, const int64_t *j_off, const int64_t *w_off)
+{
+    int64_t len = 0;
+    for (int64_t b = 0; b < B; ++b)
+        len = std::max(len, w_off[b] + (n_off[b + 1] - n_off[b]) * 2 * (j_off[b + 1] - j_off[b]));
+    return len;
+}
+
+bool non_decreasing(int64_t B, const int64_t *off)
+{
+    for (int64_t b = 0; b < B; ++b)
+        if (off[b + 1] < off[b]) return false;
+    return true;
+}
+
+// Work-queue head of one scan launch: the next of a ring of pre-zeroed counters.  (Not a memset per
+// launch: a memset is a copy-engine operation, and behind a bulk H2D copy on that engine it would hold
+// the kernel back for the whole transfer -- the reason the H2D copy of the next light curves did not
+// overlap the running scan in round 1.)
+cudaError_t next_counter(gf_handle h, int **counter)
+{
+    if (h->counter_next == N_COUNTERS) {
+        cudaError_t e = cudaMemsetAsync(h->counters, 0, N_COUNTERS * sizeof(int), h->stream);
+        if (e != cudaSuccess) return e;
+        h->counter_next = 0;
+    }
+    *counter = h->counters + h->counter_next++;
+    return cudaSuccess;
 }
 
 // Batch geometry shared by the scan entry points.
@@ -398,118 +518,187 @@ int check_geometry(gf_handle h, int64_t B, const int64_t *n_off, const int64_t *
     return GF_OK;
 }
 
-struct Timer {
-    gf_handle h;
-    explicit Timer(gf_handle h_) : h(h_) { cudaEventRecord(h->ev0, h->stream); }
-    ~Timer() { cudaEventRecord(h->ev1, h->stream); h->timed = true; }
-};
+// The argument checks of a scan, all before anything is staged; B == 0 passes them with nothing to do.
+int check_scan(gf_handle h, int mode, int64_t B, const int64_t *n_off, const int64_t *t_off,
+               const int64_t *j_off, const double *t, int64_t t_len, const double *coef, const double *ddiag,
+               const int32_t *status, uint32_t flags, Geometry *g)
+{
+    int rc = check_geometry(h, B, n_off, t_off, j_off, t_len, g);
+    if (rc != GF_OK || B == 0) return rc;
+    if (!t || !coef || !ddiag || !status) return fail(h, GF_E_ARG, "null data pointer");
+    if ((flags & GF_FLAG_SHARED_Y) && mode != gf::MODE_LOGLIKE)
+        return fail(h, GF_E_ARG, "GF_FLAG_SHARED_Y: log-likelihood only");
+    return GF_OK;
+}
+
+// The arguments of one scan launch, staged into `c`.
+gf::ScanArgs stage_scan(Call &c, const Geometry &g, int64_t B, const int64_t *n_off, const int64_t *t_off,
+                        const int64_t *j_off, const int64_t *w_off, const double *t, int64_t t_len,
+                        const double *y, const double *diag, const double *coef, const double *ddiag,
+                        uint64_t seed, uint64_t seq0, double *out_x, double *out_W, int64_t w_len,
+                        double *logdet, double *quad, int32_t *status, uint32_t flags)
+{
+    gf::ScanArgs A;
+    std::memset(&A, 0, sizeof(A));
+    A.B = B;
+    A.n_off = c.in(S_NOFF, n_off, (size_t)B + 1);
+    A.t_off = c.in(S_TOFF, t_off, (size_t)B);
+    A.j_off = c.in(S_JOFF, j_off, (size_t)B + 1);
+    A.w_off = c.in(S_WOFF, w_off, (size_t)B);
+    A.order = c.in(S_ORDER, (const int32_t *)g.order.data(), (size_t)B);
+    GF_STEP(c, next_counter(c.h, &A.counter));
+    // (the small, usually pageable arrays first: a pageable copy blocks the host until everything queued
+    // before it on the copy-in stream has been copied -- behind the bulk arrays that would be their whole
+    // transfer time)
+    A.coef = c.in(S_COEF, coef, (size_t)g.total_j * 4);
+    A.ddiag = c.in(S_DDIAG, ddiag, (size_t)B);
+    A.t = c.in(S_T, t, (size_t)t_len);
+    A.y_like_t = (flags & GF_FLAG_SHARED_Y) ? 1 : 0;
+    const size_t y_len = A.y_like_t ? (size_t)t_len : (size_t)g.total_n;
+    A.y = c.in(S_Y, y, y_len);
+    A.diag = c.in(S_DIAG, diag, y_len);
+    A.seed = seed;
+    A.seq0 = seq0;
+    // small outputs first: the caller's scalars do not wait behind the bulk copy
+    A.logdet = c.out(S_LOGDET, logdet, (size_t)B);
+    A.quad = c.out(S_QUAD, quad, (size_t)B);
+    A.status = c.out(S_STATUS, status, (size_t)B);
+    A.out_x = c.out(S_OUT, out_x, (size_t)g.total_n);
+    A.out_W = c.out(S_OUTW, out_W, (size_t)w_len);
+    // the kernels always write logdet: give them scratch when the caller does not want it
+    if (!logdet) A.logdet = (double *)c.scratch(S_LOGDET, (size_t)B * sizeof(double));
+    return A;
+}
+
+// Launch the scan kernel that serves the batch's widest state `jmax` under `flags`, record which one
+// it was (gf_last_scan_path), and return how many launches it took.
+int dispatch_scan(Call &c, int mode, const gf::ScanArgs &A, int jmax, uint32_t flags)
+{
+    gf_handle h = c.h;
+    int path, n = 1;
+    if ((flags & GF_FLAG_REFERENCE_ORDER) || jmax > GF_MAX_J) {
+        // reference order; a state wider than the register-resident kernels take (J > 176) lives
+        // in L2-resident global scratch whatever the flags
+        const int grid = (int)std::min<int64_t>(A.B, (int64_t)h->sm_count);
+        const size_t bytes = gf::scan_ref_scratch_bytes(jmax, grid);
+        void *state = bytes ? c.scratch(S_WIDE, bytes) : nullptr;
+        GF_STEP(c, gf::launch_scan_ref(mode, A, jmax, grid, (double *)state, h->stream));
+        path = bytes ? GF_PATH_WIDE : GF_PATH_REF;
+    } else if ((flags & GF_FLAG_BLOCKED) && gf::scan_blk_supports(mode, jmax)) {
+        GF_STEP(c, gf::launch_scan_blk(mode, A, h->sm_count, h->stream));
+        path = GF_PATH_BLOCKED;
+    } else if (!(flags & GF_FLAG_WIDE_KERNEL) && gf::scan_small_supports(mode, jmax)) {
+        // every sequence of the batch is narrow (J <= 32): one warp per sequence
+        GF_STEP(c, gf::launch_scan_small(mode, A, jmax, h->sm_count, h->stream, &n));
+        path = GF_PATH_SMALL;
+    } else {
+        GF_STEP(c, gf::launch_scan_fast(mode, A, jmax, h->sm_count, h->stream, &n));
+        path = GF_PATH_FAST;
+    }
+    if (c.ok()) h->scan_path = path;
+    return n;
+}
 
 int run_scan(gf_handle h, int mode, int64_t B, const int64_t *n_off, const int64_t *t_off,
              const int64_t *j_off, const int64_t *w_off, const double *t, int64_t t_len,
              const double *y, const double *diag, const double *coef, const double *ddiag,
-             uint64_t seed, uint64_t seq0, double *out_x, double *out_W, int64_t w_len,
+             uint64_t seed, uint64_t seq0, double *out_x, double *out_W,
              double *logdet, double *quad, int32_t *status, uint32_t flags)
 {
     Geometry g;
-    int rc = check_geometry(h, B, n_off, t_off, j_off, t_len, &g);
-    if (rc != GF_OK) return rc;
-    if (B == 0) return GF_OK;
-    if (!t || !coef || !ddiag || !status) return fail(h, GF_E_ARG, "null data pointer");
-    Guard guard(h->device);
+    int rc = check_scan(h, mode, B, n_off, t_off, j_off, t, t_len, coef, ddiag, status, flags, &g);
+    if (rc != GF_OK || B == 0) return rc;
+    const int64_t w_len = out_W ? w_extent(B, n_off, j_off, w_off) : 0;
+    Call c(h, flags);
+    const gf::ScanArgs A = stage_scan(c, g, B, n_off, t_off, j_off, w_off, t, t_len, y, diag, coef, ddiag,
+                                      seed, seq0, out_x, out_W, w_len, logdet, quad, status, flags);
+    c.kernels(true, [&] { return dispatch_scan(c, mode, A, g.jmax, flags); });
+    return c.finish();
+}
 
-    gf::ScanArgs A;
-    std::memset(&A, 0, sizeof(A));
-    A.B = B;
-    GF_CUDA(h, stage_in(h, S_NOFF, n_off, (size_t)B + 1, &A.n_off));
-    GF_CUDA(h, stage_in(h, S_TOFF, t_off, (size_t)B, &A.t_off));
-    GF_CUDA(h, stage_in(h, S_JOFF, j_off, (size_t)B + 1, &A.j_off));
-    if (w_off) GF_CUDA(h, stage_in(h, S_WOFF, w_off, (size_t)B, &A.w_off));
-    const int32_t *order_dev = nullptr;
-    GF_CUDA(h, stage_in(h, S_ORDER, (const int32_t *)g.order.data(), (size_t)B, &order_dev));
-    A.order = order_dev;
-    {
-        // Work-queue head of this launch: the next of a ring of pre-zeroed counters.  (Not a memset per
-        // launch: a memset is a copy-engine operation, and behind a bulk H2D copy on that engine it
-        // would hold the kernel back for the whole transfer -- the reason the H2D copy of the next
-        // light curves did not overlap the running scan in round 1.)
-        if (h->counter_next == N_COUNTERS) {
-            GF_CUDA(h, cudaMemsetAsync(h->counters, 0, N_COUNTERS * sizeof(int), h->stream));
-            h->counter_next = 0;
-        }
-        A.counter = h->counters + h->counter_next++;
+// ---- k right-hand sides per sequence on one factor ------------------------------------------
+// mode 1: samples  out[b][r][:] = L_b (sqrt(d_b) o n_{b,r});   mode 0: quad[b][r] = z^T D^-1 z, z = L_b^-1 y_{b,r}
+int run_multi(gf_handle h, int mode, int64_t B, const int64_t *n_off, const int64_t *t_off,
+              const int64_t *j_off, const double *t, int64_t t_len, const double *diag,
+              const double *coef, const double *ddiag, int64_t k, const double *in /* normals | y */,
+              uint64_t seed, uint64_t seq0, double *out, double *logdet, double *quad, int32_t *status,
+              uint32_t flags)
+{
+    if (!h) return GF_E_ARG;
+    if (k < 1) return fail(h, GF_E_ARG, "k must be >= 1");
+    Geometry g;
+    int rc = check_scan(h, gf::MODE_FACTOR, B, n_off, t_off, j_off, t, t_len, coef, ddiag, status, flags, &g);
+    if (rc != GF_OK || B == 0) return rc;
+    if (B * k > 0x7fffffff) return fail(h, GF_E_ARG, "too many right-hand sides");
+    Call c(h, flags);
+
+    // 1. the inputs the factor and the sweeps share, on the device once
+    const double *d_t = c.in(S_MT, t, (size_t)t_len);
+    const double *d_diag = c.in(S_MDIAG, diag, (size_t)g.total_n);
+    const double *d_coef = c.in(S_MCOEF, coef, (size_t)g.total_j * 4);
+    const double *d_ddiag = c.in(S_MDDIAG, ddiag, (size_t)B);
+    // 2. the factor: d[sum N], W[sum N J] in library scratch
+    std::vector<int64_t> w_off((size_t)B);
+    int64_t w_len = 0, max_n = 0;
+    for (int64_t b = 0; b < B; ++b) {
+        w_off[(size_t)b] = w_len;
+        w_len += (n_off[b + 1] - n_off[b]) * 2 * (j_off[b + 1] - j_off[b]);
+        max_n = std::max(max_n, n_off[b + 1] - n_off[b]);
     }
-    // (the small, usually pageable arrays first: a pageable copy blocks the host until everything queued
-    // before it on the copy-in stream has been copied -- behind the bulk arrays that would be their whole
-    // transfer time)
-    GF_CUDA(h, stage_in(h, S_COEF, coef, (size_t)g.total_j * 4, &A.coef));
-    GF_CUDA(h, stage_in(h, S_DDIAG, ddiag, (size_t)B, &A.ddiag));
-    GF_CUDA(h, stage_in(h, S_T, t, (size_t)t_len, &A.t));
-    const bool shared_y = (flags & GF_FLAG_SHARED_Y) != 0;
-    if (shared_y && mode != gf::MODE_LOGLIKE) return fail(h, GF_E_ARG, "GF_FLAG_SHARED_Y: log-likelihood only");
-    A.y_like_t = shared_y ? 1 : 0;
-    const size_t y_len = shared_y ? (size_t)t_len : (size_t)g.total_n;
-    GF_CUDA(h, stage_in(h, S_Y, y, y_len, &A.y));
-    GF_CUDA(h, stage_in(h, S_DIAG, diag, y_len, &A.diag));
-    A.seed = seed;
-    A.seq0 = seq0;
-
-    Out<double> o_x, o_W, o_ld, o_q;
-    Out<int32_t> o_st;
-    GF_CUDA(h, stage_out(h, S_OUT, out_x, (size_t)g.total_n, &o_x));
-    GF_CUDA(h, stage_out(h, S_OUTW, out_W, (size_t)w_len, &o_W));
-    GF_CUDA(h, stage_out(h, S_LOGDET, logdet, (size_t)B, &o_ld));
-    GF_CUDA(h, stage_out(h, S_QUAD, quad, (size_t)B, &o_q));
-    GF_CUDA(h, stage_out(h, S_STATUS, status, (size_t)B, &o_st));
-    A.out_x = o_x.dev; A.out_W = o_W.dev; A.quad = o_q.dev; A.status = o_st.dev;
-    // the kernels always write logdet: give them scratch when the caller does not want it
-    if (!o_ld.dev) {
-        void *ld = nullptr;
-        GF_CUDA(h, reserve(h, S_LOGDET, (size_t)B * sizeof(double), &ld));
-        A.logdet = (double *)ld;
+    double *d_d = (double *)c.scratch(S_MD, (size_t)std::max<int64_t>(g.total_n, 1) * sizeof(double));
+    double *d_W = (double *)c.scratch(S_MW, (size_t)std::max<int64_t>(w_len, 1) * sizeof(double));
+    const gf::ScanArgs A = stage_scan(c, g, B, n_off, t_off, j_off, w_off.data(), d_t, t_len, nullptr, d_diag,
+                                      d_coef, d_ddiag, 0, 0, d_d, d_W, w_len, logdet, nullptr, status, flags);
+    c.kernels(true, [&] { return dispatch_scan(c, gf::MODE_FACTOR, A, g.jmax, flags); });
+    // 3. virtual sequences v = b k + r: own samples, shared time stamps, factor and kernel
+    const int64_t V = B * k;
+    std::vector<int64_t> vn((size_t)V + 1), vt((size_t)V), vj((size_t)V + 1), vw((size_t)V), vd((size_t)V);
+    vn[0] = 0; vj[0] = 0;
+    for (int64_t b = 0; b < B; ++b) {
+        const int64_t N = n_off[b + 1] - n_off[b], Jc = j_off[b + 1] - j_off[b];
+        for (int64_t r = 0; r < k; ++r) {
+            const size_t v = (size_t)(b * k + r);
+            vn[v + 1] = vn[v] + N;
+            vj[v + 1] = vj[v] + Jc;
+            vt[v] = t_off[b];
+            vw[v] = w_off[(size_t)b];
+            vd[v] = n_off[b];
+        }
+    }
+    const int64_t *d_vn = c.in(S_VNOFF, (const int64_t *)vn.data(), (size_t)V + 1);
+    const int64_t *d_vt = c.in(S_VTOFF, (const int64_t *)vt.data(), (size_t)V);
+    const int64_t *d_vj = c.in(S_VJOFF, (const int64_t *)vj.data(), (size_t)V + 1);
+    const int64_t *d_vw = c.in(S_VWOFF, (const int64_t *)vw.data(), (size_t)V);
+    const int64_t *d_vd = c.in(S_VDOFF, (const int64_t *)vd.data(), (size_t)V);
+    // the coefficient rows of sequence b, k times (the sweep kernel reads CSR rows per sequence)
+    double *d_vcoef = (double *)c.scratch(S_VCOEF, (size_t)std::max<int64_t>(g.total_j * k, 1) * 4 * sizeof(double));
+    for (int64_t b = 0; b < B; ++b) {
+        const int64_t Jc = j_off[b + 1] - j_off[b];
+        for (int64_t r = 0; r < k; ++r)
+            GF_STEP(c, cudaMemcpyAsync(d_vcoef + 4 * vj[(size_t)(b * k + r)], d_coef + 4 * j_off[b],
+                                       (size_t)Jc * 4 * sizeof(double), cudaMemcpyDeviceToDevice, h->stream));
+    }
+    const size_t total_v = (size_t)g.total_n * (size_t)k;
+    const double *d_in = c.in(S_MY, in, total_v);
+    if (mode == 1) {
+        double *d_out = c.out(S_MOUT, out, total_v);
+        c.kernels(true, [&] {
+            GF_STEP(c, gf::launch_multi_prep(V, max_n, d_vn, d_vd, d_d, d_in, seed, seq0, d_out, h->stream));
+            GF_STEP(c, gf::launch_sweep(1, V, d_vn, d_vt, d_vj, d_vw, d_t, d_vcoef, d_W, d_out, d_out, g.jmax / 2,
+                                        h->stream));
+            return 2;
+        });
     } else {
-        A.logdet = o_ld.dev;
+        double *d_z = (double *)c.scratch(S_MZ, std::max<size_t>(total_v, 1) * sizeof(double));
+        double *d_quad = c.out(S_MQUAD, quad, (size_t)V);
+        c.kernels(true, [&] {
+            GF_STEP(c, gf::launch_sweep(0, V, d_vn, d_vt, d_vj, d_vw, d_t, d_vcoef, d_W, d_in, d_z, g.jmax / 2,
+                                        h->stream));
+            GF_STEP(c, gf::launch_multi_quad(V, d_vn, d_vd, d_d, d_z, d_quad, h->stream));
+            return 2;
+        });
     }
-
-    GF_CUDA(h, begin_kernel(h));
-    {
-        Timer timer(h);
-        if ((flags & GF_FLAG_REFERENCE_ORDER) || g.jmax > GF_MAX_J) {
-            // reference order; a state wider than the register-resident kernels take (J > 176) lives
-            // in L2-resident global scratch whatever the flags
-            const int grid = (int)std::min<int64_t>(B, (int64_t)h->sm_count);
-            const size_t bytes = gf::scan_ref_scratch_bytes(g.jmax, grid);
-            void *state = nullptr;
-            if (bytes) GF_CUDA(h, reserve(h, S_WIDE, bytes, &state));
-            GF_CUDA(h, gf::launch_scan_ref(mode, A, g.jmax, grid, (double *)state, h->stream));
-            h->launches += 1;
-            h->scan_path = bytes ? GF_PATH_WIDE : GF_PATH_REF;
-        } else if ((flags & GF_FLAG_BLOCKED) && gf::scan_blk_supports(mode, g.jmax)) {
-            GF_CUDA(h, gf::launch_scan_blk(mode, A, h->sm_count, h->stream));
-            h->launches += 1;
-            h->scan_path = GF_PATH_BLOCKED;
-        } else if (!(flags & GF_FLAG_WIDE_KERNEL) && gf::scan_small_supports(mode, g.jmax)) {
-            // every sequence of the batch is narrow (J <= 32): one warp per sequence
-            int n = 0;
-            GF_CUDA(h, gf::launch_scan_small(mode, A, g.jmax, h->sm_count, h->stream, &n));
-            h->launches += n;
-            h->scan_path = GF_PATH_SMALL;
-        } else {
-            int n = 0;
-            GF_CUDA(h, gf::launch_scan_fast(mode, A, g.jmax, h->sm_count, h->stream, &n));
-            h->launches += n;
-            h->scan_path = GF_PATH_FAST;
-        }
-    }
-
-    GF_CUDA(h, end_kernel(h));
-    // small outputs first: the caller's scalars do not wait behind the bulk copy
-    GF_CUDA(h, finish_out(h, o_ld));
-    GF_CUDA(h, finish_out(h, o_q));
-    GF_CUDA(h, finish_out(h, o_st));
-    GF_CUDA(h, finish_out(h, o_x));
-    GF_CUDA(h, finish_out(h, o_W));
-    GF_CUDA(h, finish_call(h, flags));
-    return GF_OK;
+    return c.finish();
 }
 
 }  // namespace
@@ -661,9 +850,8 @@ int gf_loglike_batched(gf_handle h, int64_t B, const int64_t *n_off, const int64
 {
     if (!h) return GF_E_ARG;
     if (B > 0 && (!y || !logdet || !quad)) return fail(h, GF_E_ARG, "null data pointer");
-    h->touched.clear();
     return run_scan(h, gf::MODE_LOGLIKE, B, n_off, t_off, j_off, nullptr, t, t_len, y, diag, coef,
-                    ddiag, 0, 0, nullptr, nullptr, 0, logdet, quad, status, flags);
+                    ddiag, 0, 0, nullptr, nullptr, logdet, quad, status, flags);
 }
 
 int gf_sample_batched(gf_handle h, int64_t B, const int64_t *n_off, const int64_t *t_off,
@@ -674,9 +862,8 @@ int gf_sample_batched(gf_handle h, int64_t B, const int64_t *n_off, const int64_
 {
     if (!h) return GF_E_ARG;
     if (B > 0 && !out) return fail(h, GF_E_ARG, "null output pointer");
-    h->touched.clear();
     return run_scan(h, gf::MODE_SAMPLE, B, n_off, t_off, j_off, nullptr, t, t_len, normals, diag,
-                    coef, ddiag, seed, seq0, out, nullptr, 0, logdet, nullptr, status, flags);
+                    coef, ddiag, seed, seq0, out, nullptr, logdet, nullptr, status, flags);
 }
 
 int gf_factor_batched(gf_handle h, int64_t B, const int64_t *n_off, const int64_t *t_off,
@@ -687,13 +874,8 @@ int gf_factor_batched(gf_handle h, int64_t B, const int64_t *n_off, const int64_
     if (!h) return GF_E_ARG;
     if (B > 0 && !d) return fail(h, GF_E_ARG, "null output pointer");
     if (W && !w_off) return fail(h, GF_E_ARG, "W needs w_off");
-    h->touched.clear();
-    int64_t w_len = 0;
-    if (W && B > 0 && n_off && j_off)
-        for (int64_t b = 0; b < B; ++b)
-            w_len = std::max(w_len, w_off[b] + (n_off[b + 1] - n_off[b]) * 2 * (j_off[b + 1] - j_off[b]));
     return run_scan(h, gf::MODE_FACTOR, B, n_off, t_off, j_off, W ? w_off : nullptr, t, t_len,
-                    nullptr, diag, coef, ddiag, 0, 0, d, W, w_len, logdet, nullptr, status, flags);
+                    nullptr, diag, coef, ddiag, 0, 0, d, W, logdet, nullptr, status, flags);
 }
 
 int gf_sweep_batched(gf_handle h, int op, int64_t B, const int64_t *n_off, const int64_t *t_off,
@@ -708,46 +890,34 @@ int gf_sweep_batched(gf_handle h, int op, int64_t B, const int64_t *n_off, const
     if (rc != GF_OK) return rc;
     if (B == 0) return GF_OK;
     if (!t || !coef || !W || !Y || !Z || !w_off) return fail(h, GF_E_ARG, "null data pointer");
-    Guard guard(h);
-    int64_t w_len = 0;
-    for (int64_t b = 0; b < B; ++b)
-        w_len = std::max(w_len, w_off[b] + (n_off[b + 1] - n_off[b]) * 2 * (j_off[b + 1] - j_off[b]));
-    const int64_t *d_noff, *d_toff, *d_joff, *d_woff;
-    const double *d_t, *d_coef, *d_W, *d_Y;
-    GF_CUDA(h, stage_in(h, S_NOFF, n_off, (size_t)B + 1, &d_noff));
-    GF_CUDA(h, stage_in(h, S_TOFF, t_off, (size_t)B, &d_toff));
-    GF_CUDA(h, stage_in(h, S_JOFF, j_off, (size_t)B + 1, &d_joff));
-    GF_CUDA(h, stage_in(h, S_WOFF, w_off, (size_t)B, &d_woff));
-    GF_CUDA(h, stage_in(h, S_T, t, (size_t)t_len, &d_t));
-    GF_CUDA(h, stage_in(h, S_COEF, coef, (size_t)g.total_j * 4, &d_coef));
-    GF_CUDA(h, stage_in(h, S_W, W, (size_t)w_len, &d_W));
-    Out<double> o_z;
-    // Z may alias Y: stage Y into the same slot the result is produced in
-    if (!is_device_ptr(Z)) {
-        GF_CUDA(h, stage_out(h, S_OUT, Z, (size_t)g.total_n, &o_z));
-        if (!is_device_ptr(Y)) {
-            // (on the compute stream: the buffer was acquired for it)
-            GF_CUDA(h, cudaMemcpyAsync(o_z.dev, Y, (size_t)g.total_n * sizeof(double),
-                                       cudaMemcpyHostToDevice, h->stream));
-            d_Y = o_z.dev;
-        } else {
-            d_Y = Y;
-        }
+    Call c(h, flags);
+    const int64_t *d_noff = c.in(S_NOFF, n_off, (size_t)B + 1);
+    const int64_t *d_toff = c.in(S_TOFF, t_off, (size_t)B);
+    const int64_t *d_joff = c.in(S_JOFF, j_off, (size_t)B + 1);
+    const int64_t *d_woff = c.in(S_WOFF, w_off, (size_t)B);
+    const double *d_t = c.in(S_T, t, (size_t)t_len);
+    const double *d_coef = c.in(S_COEF, coef, (size_t)g.total_j * 4);
+    const double *d_W = c.in(S_W, W, (size_t)w_extent(B, n_off, j_off, w_off));
+    // Z may alias Y: with Z on the host, a host Y goes into the buffer Z is produced in (on the compute
+    // stream: the buffer was acquired for it)
+    const bool z_on_device = is_device_ptr(Z);
+    double *d_Z = c.out(S_OUT, Z, (size_t)g.total_n);
+    const double *d_Y;
+    if (z_on_device) {
+        d_Y = c.in(S_Y, Y, (size_t)g.total_n);
+    } else if (is_device_ptr(Y)) {
+        d_Y = Y;
     } else {
-        o_z.dev = Z;
-        GF_CUDA(h, stage_in(h, S_Y, Y, (size_t)g.total_n, &d_Y));
+        GF_STEP(c, cudaMemcpyAsync(d_Z, Y, (size_t)g.total_n * sizeof(double), cudaMemcpyHostToDevice,
+                                   h->stream));
+        d_Y = d_Z;
     }
-    GF_CUDA(h, begin_kernel(h));
-    {
-        Timer timer(h);
-        GF_CUDA(h, gf::launch_sweep(op, B, d_noff, d_toff, d_joff, d_woff, d_t, d_coef, d_W, d_Y,
-                                    o_z.dev, g.jmax / 2, h->stream));
-        h->launches += 1;
-    }
-    GF_CUDA(h, end_kernel(h));
-    GF_CUDA(h, finish_out(h, o_z));
-    GF_CUDA(h, finish_call(h, flags));
-    return GF_OK;
+    c.kernels(true, [&] {
+        GF_STEP(c, gf::launch_sweep(op, B, d_noff, d_toff, d_joff, d_woff, d_t, d_coef, d_W, d_Y, d_Z,
+                                    g.jmax / 2, h->stream));
+        return 1;
+    });
+    return c.finish();
 }
 
 int gf_psd_batched(gf_handle h, int64_t B, const int64_t *j_off, const double *coef_base,
@@ -758,27 +928,18 @@ int gf_psd_batched(gf_handle h, int64_t B, const int64_t *j_off, const double *c
     if (B < 0 || F < 0) return fail(h, GF_E_ARG, "negative size");
     if (B == 0 || F == 0) return GF_OK;
     if (!j_off || !coef_base || !omega || !out) return fail(h, GF_E_ARG, "null data pointer");
-    for (int64_t b = 0; b < B; ++b)
-        if (j_off[b + 1] < j_off[b]) return fail(h, GF_E_ARG, "offsets must be non-decreasing");
-    Guard guard(h);
-    const int64_t *d_joff;
-    const double *d_coef, *d_delta, *d_omega;
-    GF_CUDA(h, stage_in(h, S_JOFF, j_off, (size_t)B + 1, &d_joff));
-    GF_CUDA(h, stage_in(h, S_COEF, coef_base, (size_t)j_off[B] * 4, &d_coef));
-    GF_CUDA(h, stage_in(h, S_DELTA, delta, (size_t)B, &d_delta));
-    GF_CUDA(h, stage_in(h, S_OMEGA, omega, (size_t)F, &d_omega));
-    Out<double> o;
-    GF_CUDA(h, stage_out(h, S_OUT, out, (size_t)B * (size_t)F, &o));
-    GF_CUDA(h, begin_kernel(h));
-    {
-        Timer timer(h);
-        GF_CUDA(h, gf::launch_psd(B, d_joff, d_coef, d_delta, d_omega, F, o.dev, h->stream));
-        h->launches += (B + 65534) / 65535;
-    }
-    GF_CUDA(h, end_kernel(h));
-    GF_CUDA(h, finish_out(h, o));
-    GF_CUDA(h, finish_call(h, flags));
-    return GF_OK;
+    if (!non_decreasing(B, j_off)) return fail(h, GF_E_ARG, "offsets must be non-decreasing");
+    Call c(h, flags);
+    const int64_t *d_joff = c.in(S_JOFF, j_off, (size_t)B + 1);
+    const double *d_coef = c.in(S_COEF, coef_base, (size_t)j_off[B] * 4);
+    const double *d_delta = c.in(S_DELTA, delta, (size_t)B);
+    const double *d_omega = c.in(S_OMEGA, omega, (size_t)F);
+    double *d_out = c.out(S_OUT, out, (size_t)B * (size_t)F);
+    c.kernels(true, [&] {
+        GF_STEP(c, gf::launch_psd(B, d_joff, d_coef, d_delta, d_omega, F, d_out, h->stream));
+        return (B + 65534) / 65535;
+    });
+    return c.finish();
 }
 
 int gf_conditional_mean(gf_handle h, int64_t N, const double *t, int64_t M, const double *ts,
@@ -791,149 +952,19 @@ int gf_conditional_mean(gf_handle h, int64_t N, const double *t, int64_t M, cons
     if (!ts || !mu || (N > 0 && (!t || !alpha)) || (Jc > 0 && !coef))
         return fail(h, GF_E_ARG, "null data pointer");
     if (Jc > 0x3fffffff) return fail(h, GF_E_ARG, "too many terms");
-    Guard guard(h);
-    const double *d_t, *d_ts, *d_coef, *d_alpha;
-    GF_CUDA(h, stage_in(h, S_T, t, (size_t)N, &d_t));
-    GF_CUDA(h, stage_in(h, S_OMEGA, ts, (size_t)M, &d_ts));
-    GF_CUDA(h, stage_in(h, S_COEF, coef, (size_t)Jc * 4, &d_coef));
-    GF_CUDA(h, stage_in(h, S_Y, alpha, (size_t)N, &d_alpha));
-    void *scratch = nullptr;
-    GF_CUDA(h, reserve(h, S_SCRATCH, (size_t)M * 2 * sizeof(double), &scratch));
-    Out<double> o;
-    GF_CUDA(h, stage_out(h, S_OUT, mu, (size_t)M, &o));
-    GF_CUDA(h, begin_kernel(h));
-    {
-        Timer timer(h);
-        GF_CUDA(h, gf::launch_cond_mean(N, d_t, M, d_ts, (int)Jc, d_coef, d_alpha,
-                                        (double *)scratch, o.dev, h->stream));
-        h->launches += 2;
-    }
-    GF_CUDA(h, end_kernel(h));
-    GF_CUDA(h, finish_out(h, o));
-    GF_CUDA(h, finish_call(h, flags));
-    return GF_OK;
+    Call c(h, flags);
+    const double *d_t = c.in(S_T, t, (size_t)N);
+    const double *d_ts = c.in(S_OMEGA, ts, (size_t)M);
+    const double *d_coef = c.in(S_COEF, coef, (size_t)Jc * 4);
+    const double *d_alpha = c.in(S_Y, alpha, (size_t)N);
+    double *scratch = (double *)c.scratch(S_SCRATCH, (size_t)M * 2 * sizeof(double));
+    double *d_mu = c.out(S_OUT, mu, (size_t)M);
+    c.kernels(true, [&] {
+        GF_STEP(c, gf::launch_cond_mean(N, d_t, M, d_ts, (int)Jc, d_coef, d_alpha, scratch, d_mu, h->stream));
+        return 2;
+    });
+    return c.finish();
 }
-
-}  // extern "C"
-
-// ---- k right-hand sides per sequence on one factor ------------------------------------------
-namespace {
-
-// mode 1: samples  out[b][r][:] = L_b (sqrt(d_b) o n_{b,r});   mode 0: quad[b][r] = z^T D^-1 z, z = L_b^-1 y_{b,r}
-int run_multi(gf_handle h, int mode, int64_t B, const int64_t *n_off, const int64_t *t_off,
-              const int64_t *j_off, const double *t, int64_t t_len, const double *diag,
-              const double *coef, const double *ddiag, int64_t k, const double *in /* normals | y */,
-              uint64_t seed, uint64_t seq0, double *out, double *logdet, double *quad, int32_t *status,
-              uint32_t flags)
-{
-    if (!h) return GF_E_ARG;
-    if (k < 1) return fail(h, GF_E_ARG, "k must be >= 1");
-    Geometry g;
-    int rc = check_geometry(h, B, n_off, t_off, j_off, t_len, &g);
-    if (rc != GF_OK) return rc;
-    if (B == 0) return GF_OK;
-    if (!t || !coef || !ddiag || !status) return fail(h, GF_E_ARG, "null data pointer");
-    if (B * k > 0x7fffffff) return fail(h, GF_E_ARG, "too many right-hand sides");
-    Guard guard(h);
-
-    // 1. the inputs the factor and the sweeps share, on the device once
-    const double *d_t, *d_diag, *d_coef, *d_ddiag;
-    GF_CUDA(h, stage_in(h, S_MT, t, (size_t)t_len, &d_t));
-    GF_CUDA(h, stage_in(h, S_MDIAG, diag, (size_t)g.total_n, &d_diag));
-    GF_CUDA(h, stage_in(h, S_MCOEF, coef, (size_t)g.total_j * 4, &d_coef));
-    GF_CUDA(h, stage_in(h, S_MDDIAG, ddiag, (size_t)B, &d_ddiag));
-    // 2. the factor: d[sum N], W[sum N J] in library scratch
-    std::vector<int64_t> w_off((size_t)B);
-    int64_t w_len = 0, max_n = 0;
-    for (int64_t b = 0; b < B; ++b) {
-        w_off[(size_t)b] = w_len;
-        w_len += (n_off[b + 1] - n_off[b]) * 2 * (j_off[b + 1] - j_off[b]);
-        max_n = std::max(max_n, n_off[b + 1] - n_off[b]);
-    }
-    void *d_d = nullptr, *d_W = nullptr;
-    GF_CUDA(h, reserve(h, S_MD, (size_t)std::max<int64_t>(g.total_n, 1) * sizeof(double), &d_d));
-    GF_CUDA(h, reserve(h, S_MW, (size_t)std::max<int64_t>(w_len, 1) * sizeof(double), &d_W));
-    std::vector<Buf *> mine = h->touched;      // run_scan's end_kernel stamps and clears the list
-    rc = run_scan(h, gf::MODE_FACTOR, B, n_off, t_off, j_off, w_off.data(), d_t, t_len, nullptr, d_diag,
-                  d_coef, d_ddiag, 0, 0, (double *)d_d, (double *)d_W, w_len, logdet, nullptr, status,
-                  flags | GF_FLAG_ASYNC);
-    if (rc != GF_OK) return rc;
-    h->touched = mine;
-    // 3. virtual sequences v = b k + r: own samples, shared time stamps, factor and kernel
-    const int64_t V = B * k;
-    std::vector<int64_t> vn((size_t)V + 1), vt((size_t)V), vj((size_t)V + 1), vw((size_t)V), vd((size_t)V);
-    std::vector<double> vcoef;
-    vcoef.reserve((size_t)g.total_j * 4 * (size_t)k);
-    vn[0] = 0; vj[0] = 0;
-    for (int64_t b = 0; b < B; ++b) {
-        const int64_t N = n_off[b + 1] - n_off[b], Jc = j_off[b + 1] - j_off[b];
-        for (int64_t r = 0; r < k; ++r) {
-            const size_t v = (size_t)(b * k + r);
-            vn[v + 1] = vn[v] + N;
-            vj[v + 1] = vj[v] + Jc;
-            vt[v] = t_off[b];
-            vw[v] = w_off[(size_t)b];
-            vd[v] = n_off[b];
-        }
-    }
-    const int64_t *d_vn, *d_vt, *d_vj, *d_vw, *d_vd;
-    const double *d_vcoef = nullptr;
-    GF_CUDA(h, stage_in(h, S_VNOFF, (const int64_t *)vn.data(), (size_t)V + 1, &d_vn));
-    GF_CUDA(h, stage_in(h, S_VTOFF, (const int64_t *)vt.data(), (size_t)V, &d_vt));
-    GF_CUDA(h, stage_in(h, S_VJOFF, (const int64_t *)vj.data(), (size_t)V + 1, &d_vj));
-    GF_CUDA(h, stage_in(h, S_VWOFF, (const int64_t *)vw.data(), (size_t)V, &d_vw));
-    GF_CUDA(h, stage_in(h, S_VDOFF, (const int64_t *)vd.data(), (size_t)V, &d_vd));
-    {
-        // the coefficient rows of sequence b, k times (the sweep kernel reads CSR rows per sequence)
-        void *p = nullptr;
-        GF_CUDA(h, reserve(h, S_VCOEF, (size_t)std::max<int64_t>(g.total_j * k, 1) * 4 * sizeof(double), &p));
-        for (int64_t b = 0; b < B; ++b) {
-            const int64_t Jc = j_off[b + 1] - j_off[b];
-            for (int64_t r = 0; r < k; ++r)
-                GF_CUDA(h, cudaMemcpyAsync((double *)p + 4 * vj[(size_t)(b * k + r)], d_coef + 4 * j_off[b],
-                                           (size_t)Jc * 4 * sizeof(double), cudaMemcpyDeviceToDevice, h->stream));
-        }
-        d_vcoef = (const double *)p;
-    }
-    const size_t total_v = (size_t)g.total_n * (size_t)k;
-    const double *d_in = nullptr;
-    GF_CUDA(h, stage_in(h, S_MY, in, total_v, &d_in));
-    if (mode == 1) {
-        Out<double> o;
-        GF_CUDA(h, stage_out(h, S_MOUT, out, total_v, &o));
-        if (o.host) h->touched.push_back(o.buf);
-        GF_CUDA(h, begin_kernel(h));
-        {
-            Timer timer(h);
-            GF_CUDA(h, gf::launch_multi_prep(V, max_n, d_vn, d_vd, (const double *)d_d, d_in, seed, seq0, o.dev, h->stream));
-            GF_CUDA(h, gf::launch_sweep(1, V, d_vn, d_vt, d_vj, d_vw, d_t, d_vcoef, (const double *)d_W, o.dev, o.dev, g.jmax / 2, h->stream));
-            h->launches += 2;
-        }
-        GF_CUDA(h, end_kernel(h));
-        GF_CUDA(h, finish_out(h, o));
-    } else {
-        void *d_z = nullptr;
-        GF_CUDA(h, reserve(h, S_MZ, std::max<size_t>(total_v, 1) * sizeof(double), &d_z));
-        Out<double> oq;
-        GF_CUDA(h, stage_out(h, S_MQUAD, quad, (size_t)V, &oq));
-        if (oq.host) h->touched.push_back(oq.buf);
-        GF_CUDA(h, begin_kernel(h));
-        {
-            Timer timer(h);
-            GF_CUDA(h, gf::launch_sweep(0, V, d_vn, d_vt, d_vj, d_vw, d_t, d_vcoef, (const double *)d_W, d_in, (double *)d_z, g.jmax / 2, h->stream));
-            GF_CUDA(h, gf::launch_multi_quad(V, d_vn, d_vd, (const double *)d_d, (const double *)d_z, oq.dev, h->stream));
-            h->launches += 2;
-        }
-        GF_CUDA(h, end_kernel(h));
-        GF_CUDA(h, finish_out(h, oq));
-    }
-    GF_CUDA(h, finish_call(h, flags));
-    return GF_OK;
-}
-
-}  // namespace
-
-extern "C" {
 
 int gf_sample_multi(gf_handle h, int64_t B, const int64_t *n_off, const int64_t *t_off,
                     const int64_t *j_off, const double *t, int64_t t_len, const double *diag,
@@ -958,9 +989,6 @@ int gf_loglike_multi(gf_handle h, int64_t B, const int64_t *n_off, const int64_t
                      logdet, quad, status, flags);
 }
 
-}  // extern "C"
-
-extern "C" {
 
 int gf_power_spectrum_batched(gf_handle h, int64_t B, int64_t N, const double *flux, double d,
                               int include_zero, double *power, uint32_t flags)
@@ -970,26 +998,18 @@ int gf_power_spectrum_batched(gf_handle h, int64_t B, int64_t N, const double *f
     if (B == 0 || N == 0) return GF_OK;
     if (!flux || !power) return fail(h, GF_E_ARG, "null data pointer");
     if (N > 0x7fffffff || B > 0x7fffffff) return fail(h, GF_E_ARG, "too large for one cuFFT plan");
-    Guard guard(h);
+    Call c(h, flags);
     if (!h->fft) h->fft = gf::new_fft_plan();
     const int64_t NC = N / 2 + 1, nout = NC - (include_zero ? 0 : 1);
-    const double *d_flux;
-    GF_CUDA(h, stage_in(h, S_FLUX, flux, (size_t)(B * N), &d_flux));
-    void *spec = nullptr;
-    GF_CUDA(h, reserve(h, S_SPEC, (size_t)(B * NC) * sizeof(double2), &spec));
-    Out<double> o;
-    GF_CUDA(h, stage_out(h, S_POWER, power, (size_t)(B * nout), &o));
-    if (o.host) h->touched.push_back(o.buf);
-    GF_CUDA(h, begin_kernel(h));
-    {
-        Timer timer(h);
-        GF_CUDA(h, gf::launch_obs_power(h->fft, B, N, d_flux, d, include_zero, (double2 *)spec, o.dev, h->stream));
-        h->launches += 1;      // our normalisation kernel (the transform is cuFFT's)
-    }
-    GF_CUDA(h, end_kernel(h));
-    GF_CUDA(h, finish_out(h, o));
-    GF_CUDA(h, finish_call(h, flags));
-    return GF_OK;
+    const double *d_flux = c.in(S_FLUX, flux, (size_t)(B * N));
+    double2 *spec = (double2 *)c.scratch(S_SPEC, (size_t)(B * NC) * sizeof(double2));
+    double *d_power = c.out(S_POWER, power, (size_t)(B * nout));
+    // one launch: our normalisation kernel (the transform is cuFFT's)
+    c.kernels(true, [&] {
+        GF_STEP(c, gf::launch_obs_power(h->fft, B, N, d_flux, d, include_zero, spec, d_power, h->stream));
+        return 1;
+    });
+    return c.finish();
 }
 
 int gf_bin_power_batched(gf_handle h, int64_t B, int64_t F, int64_t nb, const int64_t *lo,
@@ -1003,29 +1023,18 @@ int gf_bin_power_batched(gf_handle h, int64_t B, int64_t F, int64_t nb, const in
     for (int64_t k = 0; k < nb; ++k)
         if (lo[k] < 0 || cnt[k] < 0 || lo[k] + cnt[k] > F) return fail(h, GF_E_ARG, "bin range outside the axis");
     if (!(constant > 0.0)) return fail(h, GF_E_ARG, "constant must be positive");
-    Guard guard(h);
-    const int64_t *d_lo, *d_cnt;
-    const double *d_axis, *d_power;
-    GF_CUDA(h, stage_in(h, S_BLO, lo, (size_t)nb, &d_lo));
-    GF_CUDA(h, stage_in(h, S_BCNT, cnt, (size_t)nb, &d_cnt));
-    GF_CUDA(h, stage_in(h, S_BAXIS, axis, (size_t)F, &d_axis));
-    GF_CUDA(h, stage_in(h, S_POWER, power, (size_t)(B * F), &d_power));
-    Out<double> os, oe;
-    GF_CUDA(h, stage_out(h, S_BSTAT, stat, (size_t)(B * nb), &os));
-    GF_CUDA(h, stage_out(h, S_BERR, err, (size_t)(B * nb), &oe));
-    if (os.host) h->touched.push_back(os.buf);
-    if (oe.host) h->touched.push_back(oe.buf);
-    GF_CUDA(h, begin_kernel(h));
-    {
-        Timer timer(h);
-        GF_CUDA(h, gf::launch_bin_power(B, F, nb, d_lo, d_cnt, d_axis, d_power, constant, os.dev, oe.dev, h->stream));
-        h->launches += 1;
-    }
-    GF_CUDA(h, end_kernel(h));
-    GF_CUDA(h, finish_out(h, os));
-    GF_CUDA(h, finish_out(h, oe));
-    GF_CUDA(h, finish_call(h, flags));
-    return GF_OK;
+    Call c(h, flags);
+    const int64_t *d_lo = c.in(S_BLO, lo, (size_t)nb);
+    const int64_t *d_cnt = c.in(S_BCNT, cnt, (size_t)nb);
+    const double *d_axis = c.in(S_BAXIS, axis, (size_t)F);
+    const double *d_power = c.in(S_POWER, power, (size_t)(B * F));
+    double *d_stat = c.out(S_BSTAT, stat, (size_t)(B * nb));
+    double *d_err = c.out(S_BERR, err, (size_t)(B * nb));
+    c.kernels(true, [&] {
+        GF_STEP(c, gf::launch_bin_power(B, F, nb, d_lo, d_cnt, d_axis, d_power, constant, d_stat, d_err, h->stream));
+        return 1;
+    });
+    return c.finish();
 }
 
 int gf_feed_stars(gf_handle h, int64_t B, const double *mass, const double *radius, const double *temperature,
@@ -1042,7 +1051,7 @@ int gf_feed_stars(gf_handle h, int64_t B, const double *mass, const double *radi
     if (!mass || !radius || !temperature || !luminosity || !delta || !coef || !ddiag ||
         (n_gran > 0 && !gran) || (n_modes > 0 && !modes))
         return fail(h, GF_E_ARG, "null data pointer");
-    Guard guard(h);
+    Call c(h, flags);
     const int nt = (int)(n_gran + n_modes);
     gf::FeedArgs A;
     std::memset(&A, 0, sizeof(A));
@@ -1055,51 +1064,43 @@ int gf_feed_stars(gf_handle h, int64_t B, const double *mass, const double *radi
     A.amp_huber_sun = std::pow(1.0, 0.886) / (std::pow(1.0, 1.89) * 5777.0 * std::pow(5777.0 / 5934.0, 0.8));
     A.gran_power_sun = 1.0 / (1.0 * std::pow(5777.0, 5.5));
     A.tau_sun = 1.0 / (1.0 * std::pow(5777.0, 3.5));
-    GF_CUDA(h, stage_in(h, S_FM, mass, (size_t)B, &A.mass));
-    GF_CUDA(h, stage_in(h, S_FR, radius, (size_t)B, &A.radius));
-    GF_CUDA(h, stage_in(h, S_FT, temperature, (size_t)B, &A.temperature));
-    GF_CUDA(h, stage_in(h, S_FL, luminosity, (size_t)B, &A.luminosity));
-    GF_CUDA(h, stage_in(h, S_FALPHA, alpha, (size_t)B, &A.alpha));
-    GF_CUDA(h, stage_in(h, S_DELTA, delta, (size_t)B, &A.delta));
-    GF_CUDA(h, stage_in(h, S_FGRAN, gran, (size_t)n_gran * 3, &A.gran));
-    GF_CUDA(h, stage_in(h, S_FMODES, modes, (size_t)n_modes * (size_t)(4 + n_gran), &A.modes));
-    void *sho_all = nullptr, *keep_all = nullptr, *count = nullptr;
-    GF_CUDA(h, reserve(h, S_FSHOALL, (size_t)B * nt * 3 * sizeof(double), &sho_all));
-    GF_CUDA(h, reserve(h, S_FKEEP, (size_t)B * nt, &keep_all));
-    GF_CUDA(h, reserve(h, S_FCOUNT, (size_t)B * sizeof(int32_t), &count));
-    GF_CUDA(h, begin_kernel(h));
-    GF_CUDA(h, gf::launch_feed_hyper(A, (double *)sho_all, (unsigned char *)keep_all, (int32_t *)count, h->stream));
-    h->launches += 1;
+    A.mass = c.in(S_FM, mass, (size_t)B);
+    A.radius = c.in(S_FR, radius, (size_t)B);
+    A.temperature = c.in(S_FT, temperature, (size_t)B);
+    A.luminosity = c.in(S_FL, luminosity, (size_t)B);
+    A.alpha = c.in(S_FALPHA, alpha, (size_t)B);
+    A.delta = c.in(S_DELTA, delta, (size_t)B);
+    A.gran = c.in(S_FGRAN, gran, (size_t)n_gran * 3);
+    A.modes = c.in(S_FMODES, modes, (size_t)n_modes * (size_t)(4 + n_gran));
+    double *sho_all = (double *)c.scratch(S_FSHOALL, (size_t)B * nt * 3 * sizeof(double));
+    unsigned char *keep_all = (unsigned char *)c.scratch(S_FKEEP, (size_t)B * nt);
+    int32_t *count = (int32_t *)c.scratch(S_FCOUNT, (size_t)B * sizeof(int32_t));
+    c.kernels(false, [&] {
+        GF_STEP(c, gf::launch_feed_hyper(A, sho_all, keep_all, count, h->stream));
+        return 1;
+    });
     // the CSR offsets are a host array of the ABI: terms kept per star back to the host, prefix sum here
     std::vector<int32_t> cnt((size_t)B);
-    GF_CUDA(h, cudaMemcpyAsync(cnt.data(), count, (size_t)B * sizeof(int32_t), cudaMemcpyDeviceToHost, h->stream));
-    GF_CUDA(h, cudaStreamSynchronize(h->stream));
+    GF_STEP(c, cudaMemcpyAsync(cnt.data(), count, (size_t)B * sizeof(int32_t), cudaMemcpyDeviceToHost, h->stream));
+    GF_STEP(c, cudaStreamSynchronize(h->stream));
+    if (!c.ok()) return c.finish();
     for (int64_t b = 0; b < B; ++b) {
         if (cnt[(size_t)b] < 0) return fail(h, GF_E_ARG, "a scaled term is overdamped (Q < 0.5): build that kernel per star");
         j_off[b + 1] = j_off[b] + cnt[(size_t)b];
     }
     const int64_t total = j_off[B];
     if (total > cap_terms) return fail(h, GF_E_ARG, "coefficient arrays too small (cap_terms)");
-    const int64_t *d_joff;
-    GF_CUDA(h, stage_in(h, S_JOFF, (const int64_t *)j_off, (size_t)B + 1, &d_joff));
-    Out<double> o_sho, o_coef, o_base, o_dd;
-    GF_CUDA(h, stage_out(h, S_FSHO, sho, (size_t)total * 3, &o_sho));
-    GF_CUDA(h, stage_out(h, S_OUT, coef, (size_t)total * 4, &o_coef));
-    GF_CUDA(h, stage_out(h, S_FBASE, base, (size_t)total * 4, &o_base));
-    GF_CUDA(h, stage_out(h, S_FDDIAG, ddiag, (size_t)B, &o_dd));
-    GF_CUDA(h, begin_kernel(h));
-    if (total > 0 || B > 0) {
-        GF_CUDA(h, gf::launch_feed_coef(A, (const double *)sho_all, (const unsigned char *)keep_all, d_joff,
-                                        o_sho.dev, o_coef.dev, o_base.dev, o_dd.dev, h->stream));
-        h->launches += 1;
-    }
-    GF_CUDA(h, end_kernel(h));
-    GF_CUDA(h, finish_out(h, o_dd));
-    GF_CUDA(h, finish_out(h, o_sho));
-    GF_CUDA(h, finish_out(h, o_coef));
-    GF_CUDA(h, finish_out(h, o_base));
-    GF_CUDA(h, finish_call(h, flags));
-    return GF_OK;
+    const int64_t *d_joff = c.in(S_JOFF, (const int64_t *)j_off, (size_t)B + 1);
+    // small outputs first
+    double *d_dd = c.out(S_FDDIAG, ddiag, (size_t)B);
+    double *d_sho = c.out(S_FSHO, sho, (size_t)total * 3);
+    double *d_coef = c.out(S_OUT, coef, (size_t)total * 4);
+    double *d_base = c.out(S_FBASE, base, (size_t)total * 4);
+    c.kernels(false, [&] {
+        GF_STEP(c, gf::launch_feed_coef(A, sho_all, keep_all, d_joff, d_sho, d_coef, d_base, d_dd, h->stream));
+        return 1;
+    });
+    return c.finish();
 }
 
 int gf_feed_sho(gf_handle h, int64_t B, const int64_t *j_off, const double *sho, const double *delta,
@@ -1110,37 +1111,28 @@ int gf_feed_sho(gf_handle h, int64_t B, const int64_t *j_off, const double *sho,
     if (B == 0) return GF_OK;
     if (!j_off || !sho || !delta || !coef || !ddiag) return fail(h, GF_E_ARG, "null data pointer");
     if (j_off[0] != 0) return fail(h, GF_E_ARG, "offsets must start at 0");
-    for (int64_t b = 0; b < B; ++b)
-        if (j_off[b + 1] < j_off[b]) return fail(h, GF_E_ARG, "offsets must be non-decreasing");
+    if (!non_decreasing(B, j_off)) return fail(h, GF_E_ARG, "offsets must be non-decreasing");
     const int64_t total = j_off[B];
-    Guard guard(h);
-    const int64_t *d_joff;
-    const double *d_sho, *d_delta;
-    GF_CUDA(h, stage_in(h, S_JOFF, j_off, (size_t)B + 1, &d_joff));
-    GF_CUDA(h, stage_in(h, S_FSHOALL, sho, (size_t)total * 3, &d_sho));
-    GF_CUDA(h, stage_in(h, S_DELTA, delta, (size_t)B, &d_delta));
-    void *dterm = nullptr, *over = nullptr;
-    GF_CUDA(h, reserve(h, S_FKEEP, (size_t)std::max<int64_t>(total, 1) * sizeof(double), &dterm));
-    GF_CUDA(h, reserve(h, S_FCOUNT, sizeof(int32_t), &over));
-    Out<double> o_coef, o_base, o_dd;
-    GF_CUDA(h, stage_out(h, S_OUT, coef, (size_t)total * 4, &o_coef));
-    GF_CUDA(h, stage_out(h, S_FBASE, base, (size_t)total * 4, &o_base));
-    GF_CUDA(h, stage_out(h, S_FDDIAG, ddiag, (size_t)B, &o_dd));
-    GF_CUDA(h, begin_kernel(h));
-    GF_CUDA(h, cudaMemsetAsync(over, 0, sizeof(int32_t), h->stream));
-    GF_CUDA(h, gf::launch_feed_sho(B, d_joff, d_sho, d_delta, o_coef.dev, o_base.dev, (double *)dterm, o_dd.dev,
-                                   (int32_t *)over, h->stream));
-    h->launches += 1;
-    GF_CUDA(h, end_kernel(h));
+    Call c(h, flags);
+    const int64_t *d_joff = c.in(S_JOFF, j_off, (size_t)B + 1);
+    const double *d_sho = c.in(S_FSHOALL, sho, (size_t)total * 3);
+    const double *d_delta = c.in(S_DELTA, delta, (size_t)B);
+    double *dterm = (double *)c.scratch(S_FKEEP, (size_t)std::max<int64_t>(total, 1) * sizeof(double));
+    int32_t *over = (int32_t *)c.scratch(S_FCOUNT, sizeof(int32_t));
+    // small outputs first
+    double *d_dd = c.out(S_FDDIAG, ddiag, (size_t)B);
+    double *d_coef = c.out(S_OUT, coef, (size_t)total * 4);
+    double *d_base = c.out(S_FBASE, base, (size_t)total * 4);
+    c.kernels(false, [&] {
+        GF_STEP(c, cudaMemsetAsync(over, 0, sizeof(int32_t), h->stream));
+        GF_STEP(c, gf::launch_feed_sho(B, d_joff, d_sho, d_delta, d_coef, d_base, dterm, d_dd, over, h->stream));
+        return 1;
+    });
     int32_t n_over = 0;
-    GF_CUDA(h, cudaMemcpyAsync(&n_over, over, sizeof(int32_t), cudaMemcpyDeviceToHost, h->stream));
-    GF_CUDA(h, cudaStreamSynchronize(h->stream));
-    if (n_over) return fail(h, GF_E_ARG, "overdamped term (Q < 0.5): build that kernel per star");
-    GF_CUDA(h, finish_out(h, o_dd));
-    GF_CUDA(h, finish_out(h, o_coef));
-    GF_CUDA(h, finish_out(h, o_base));
-    GF_CUDA(h, finish_call(h, flags));
-    return GF_OK;
+    GF_STEP(c, cudaMemcpyAsync(&n_over, over, sizeof(int32_t), cudaMemcpyDeviceToHost, h->stream));
+    GF_STEP(c, cudaStreamSynchronize(h->stream));
+    if (c.ok() && n_over) return fail(h, GF_E_ARG, "overdamped term (Q < 0.5): build that kernel per star");
+    return c.finish();
 }
 
 int gf_bandpass_amplitude(gf_handle h, int64_t B, const double *temperature, int64_t n_wl, const double *wl_um,
@@ -1150,20 +1142,16 @@ int gf_bandpass_amplitude(gf_handle h, int64_t B, const double *temperature, int
     if (B < 0 || n_wl < 0) return fail(h, GF_E_ARG, "negative size");
     if (B == 0) return GF_OK;
     if (!temperature || !wl_um || !transmittance || !out || n_wl < 2) return fail(h, GF_E_ARG, "null data pointer");
-    Guard guard(h);
-    const double *d_T, *d_wl, *d_f;
-    GF_CUDA(h, stage_in(h, S_FT, temperature, (size_t)B, &d_T));
-    GF_CUDA(h, stage_in(h, S_FWL, wl_um, (size_t)n_wl, &d_wl));
-    GF_CUDA(h, stage_in(h, S_FFILT, transmittance, (size_t)n_wl, &d_f));
-    Out<double> o;
-    GF_CUDA(h, stage_out(h, S_OUT, out, (size_t)B, &o));
-    GF_CUDA(h, begin_kernel(h));
-    GF_CUDA(h, gf::launch_bandpass(B, d_T, n_wl, d_wl, d_f, o.dev, h->stream));
-    h->launches += 1;
-    GF_CUDA(h, end_kernel(h));
-    GF_CUDA(h, finish_out(h, o));
-    GF_CUDA(h, finish_call(h, flags));
-    return GF_OK;
+    Call c(h, flags);
+    const double *d_T = c.in(S_FT, temperature, (size_t)B);
+    const double *d_wl = c.in(S_FWL, wl_um, (size_t)n_wl);
+    const double *d_f = c.in(S_FFILT, transmittance, (size_t)n_wl);
+    double *d_out = c.out(S_OUT, out, (size_t)B);
+    c.kernels(false, [&] {
+        GF_STEP(c, gf::launch_bandpass(B, d_T, n_wl, d_wl, d_f, d_out, h->stream));
+        return 1;
+    });
+    return c.finish();
 }
 
 }  // extern "C"
